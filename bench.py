@@ -10,11 +10,13 @@ target update) -- PathPlan_City.run_thread_OffPolicy + update (Envs/PathPlan_Cit
 
   python bench.py --gpus N --steps K --warmup W            (N > 1: launched by torchrun, one rank per GPU)
   python bench.py --impl reference ...                     (the CPU arm: the oracle port on the host threads)
+  python bench.py ... --dump-outputs DIR                   (also write what the last timed step computed, DIR/<name>.npy)
 
 Prints ONE JSON line (rank 0).
-  value      whole-job env steps/s, inputs resident in HBM.  The K-step block (barrier + synchronize on both sides, CUDA
-             events, max over ranks) is REPEATED until the timed region is >= --min-seconds; value comes from the median block
-             (`repeats`, `block_ms_*` are printed), so the region is long enough for the clock sampler and the driver to see.
+  value      whole-job env steps/s, inputs resident in HBM.  After W warm-up steps, exactly K steps are timed as one block
+             (barrier + synchronize on both sides, CUDA events, max over ranks); the default K makes that window about 1 s on
+             one B200 at the default workload.  --dump-outputs writes the state right after this block, before anything below
+             runs, so it depends on the arguments alone.  The measurements below keep their own bounded step counts.
   e2e        the same iteration through the reference-facing plug-in classes (PathPlan_City_B200 / DQN_Trainer_B200 built
              from the XML configs) with HOST arrays at every boundary, H2D/D2H inside the timed region.
   roofline   dominant kernel: algorithmic bytes|flops / CUDA-event time vs MEASURED_PEAKS.json.
@@ -54,7 +56,8 @@ PYTHON_REFERENCE = {"value": 100.0, "unit": "env_steps/s", "cores": 1, "kind": "
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps of the headline loop (default 25000: about 1 s at 45 us per step on one B200; 200 with --impl reference)")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--envs", type=int, default=4096, help="envs per GPU (BASELINE configs[1])")
@@ -72,8 +75,8 @@ def parse():
     ap.add_argument("--fuse", type=int, default=0, help="1 = get_action + env step as one kernel on the tensor-core path, 0 = two PDL-chained kernels (default, faster)")
     ap.add_argument("--fuse-dw", type=int, default=-1, help="1 = optimiser step inside the weight-gradient kernel (uavrl_set_fuse_dw_adam), 0 = separate kernel, -1 = library default")
     ap.add_argument("--per", type=int, default=0, help="1 = prioritised replay (device SumTree equivalent) instead of uniform sampling")
-    ap.add_argument("--min-seconds", type=float, default=1.0, help="the K-step block is repeated until the timed region is at least this long")
-    ap.add_argument("--max-repeats", type=int, default=4000)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the env state, observations and learner state of the last step as DIR/<name>.npy")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the sub-results for the other BASELINE configs")
@@ -253,23 +256,17 @@ def run_reference_arm(a):
     loop, nthreads = make_oracle_loop(a, a.envs, a.threads)
     for _ in range(max(a.warmup, 2)):
         loop.iteration(a.eps)
-    # the K-step block repeated like the GPU arm (median block), bounded to about --cpu-seconds x 3 of work
-    blocks, t_all0 = [], time.perf_counter()
-    while len(blocks) < 3 or (time.perf_counter() - t_all0 < 3 * a.cpu_seconds and len(blocks) < 9):
-        t0 = time.perf_counter()
-        for _ in range(a.steps):
-            loop.iteration(a.eps)
-        blocks.append(time.perf_counter() - t0)
-        if time.perf_counter() - t_all0 > 6 * a.cpu_seconds:
-            break
-    dt = statistics.median(blocks)
+    t0 = time.perf_counter()
+    for _ in range(a.steps):
+        loop.iteration(a.eps)
+    dt = time.perf_counter() - t0
     v = a.envs * a.steps / dt
     sample = ("each step = one lockstep iteration of %d envs + 1 %s update (batch %d) on the oracle port, %d OpenMP threads "
               "(C restatement of the Python reference; the Python reference itself cannot travel to the GPU box); "
-              "median of %d blocks of %d steps" % (a.envs, a.algo.upper(), a.batch, nthreads, len(blocks), a.steps))
+              "%d timed steps" % (a.envs, a.algo.upper(), a.batch, nthreads, a.steps))
     out = {"impl": "reference", "metric": "env steps/sec (+ DQN updates/sec), 500x500x100 city", "value": v,
            "unit": "env_steps/s", "updates_per_s": a.steps / dt, "n_gpus": a.gpus, "steps": a.steps, "warmup": a.warmup,
-           "repeats": len(blocks), "block_s": blocks,
+           "timed_region_s": dt,
            "ms_per_step": 1e3 * dt / a.steps, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
            "dtype": "f64 env / f32 learner", "data": "synthetic", "config": config_dict(a, 1),
            "cpu_baseline": {"value": v, "unit": "env_steps/s", "cores": nthreads, "kind": "port", "sample": sample,
@@ -332,44 +329,54 @@ class Workload:
         self.L.close(); self.env.close()
 
 
-def timed_blocks(wl, a, dev, local, stream, barrier, sampler=None):
-    """Repeat the K-step block (barrier + synchronize on both sides, CUDA events on the launching stream) until the timed
-    region is >= --min-seconds.  Returns per-block ms (max over ranks), wall seconds of the region, sampler mark."""
+def timed_steps(wl, a, dev, stream, barrier, sampler=None):
+    """The K = --steps timed steps as one block: barrier + synchronize on both sides, CUDA events on the launching stream.
+    Returns the block's ms (max over ranks), wall seconds of the region, sampler mark."""
     import torch
     world, dist = wl.world, wl.dist
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    # pilot block: decides the repeat count (same on every rank)
-    barrier()
-    e0.record(stream); wl.iterate(a.steps); e1.record(stream)
-    barrier()
-    pilot = torch.tensor([e0.elapsed_time(e1)], device=dev, dtype=torch.float64)
-    if world > 1:
-        dist.all_reduce(pilot, op=dist.ReduceOp.MAX)
-    repeats = int(min(a.max_repeats, max(3, np.ceil(a.min_seconds * 1e3 / max(float(pilot.item()), 1e-3)))))
-    evs = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(repeats)]
     mark = sampler.mark() if sampler else 0
     barrier()
     t0 = time.perf_counter()
-    for s, e in evs:
-        s.record(stream)
-        wl.iterate(a.steps)
-        e.record(stream)
-        barrier()                                   # barrier + synchronize: the block is bracketed on both sides
+    e0.record(stream)
+    wl.iterate(a.steps)
+    e1.record(stream)
+    barrier()
     wall = time.perf_counter() - t0
-    ms = torch.tensor([s.elapsed_time(e) for s, e in evs], device=dev, dtype=torch.float64)
+    ms = torch.tensor([e0.elapsed_time(e1)], device=dev, dtype=torch.float64)
     if world > 1:
-        dist.all_reduce(ms, op=dist.ReduceOp.MAX)   # every block: max over ranks
-    return ms.cpu().numpy(), wall, mark
+        dist.all_reduce(ms, op=dist.ReduceOp.MAX)
+    return float(ms.item()), wall, mark
+
+
+def dump_outputs(wl, out_dir, max_envs=1 << 16):
+    """What a caller of the timed loop receives after its last step, as float32/float64 .npy files: this rank's env state
+    (the step's reward, done flags, fp64 kinematics, counters) and observations, and the learner's parameters, Adam moments
+    and last gradient.  Batches above max_envs are cut to a fixed seeded sample of envs (env_index.npy), which keeps the
+    files well under 64 MB."""
+    os.makedirs(out_dir, exist_ok=True)
+    st = wl.env.get_state()
+    st["obs"] = wl.env.observe().cpu().numpy()
+    n = wl.env.n
+    rows = np.arange(n) if n <= max_envs else np.sort(np.random.default_rng(0).choice(n, max_envs, replace=False))
+    arrays = {"env_index": rows.astype(np.float64)}
+    for k, v in st.items():
+        v = v[rows]
+        arrays["env_" + k] = v if v.dtype in (np.float32, np.float64) else v.astype(np.float64)
+    for which, k in enumerate(("q_local", "q_target", "adam_exp_avg", "adam_exp_avg_sq", "grad")):
+        arrays["learner_" + k] = wl.L.get_params(which)
+    arrays["learner_counters"] = np.array(wl.L.counters(), np.float64)          # epoch, Adam step
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
 
 
 def measure_config(a_sub, rank, world, local, dist, dev, stream, barrier, label):
     """One sub-result (another BASELINE config) with the same timing discipline; returns a small dict (rank 0) or None."""
     wl = Workload(a_sub, rank, world, local, dist)
     wl.iterate(max(a_sub.warmup, 3))
-    ms, wall, _ = timed_blocks(wl, a_sub, dev, local, stream, barrier)
-    med = float(np.median(ms))
-    out = {"label": label, "value": a_sub.envs * world * a_sub.steps / (med * 1e-3), "unit": "env_steps/s",
-           "updates_per_s": a_sub.steps / (med * 1e-3), "ms_per_step": med / a_sub.steps, "repeats": int(len(ms)),
+    ms, wall, _ = timed_steps(wl, a_sub, dev, stream, barrier)
+    out = {"label": label, "value": a_sub.envs * world * a_sub.steps / (ms * 1e-3), "unit": "env_steps/s",
+           "updates_per_s": a_sub.steps / (ms * 1e-3), "ms_per_step": ms / a_sub.steps,
            "timed_region_s": wall, "n_gpus": world, "config": config_dict(a_sub, world), "tensor_cores": bool(wl.tc_on)}
     wl.close()
     return out if rank == 0 else None
@@ -511,10 +518,11 @@ def run_ours(a):
     torch.cuda.synchronize(dev)
 
     launches0 = _lib.launch_count()
-    ms_blocks, t_wall, mark = timed_blocks(wl, a, dev, local, stream, barrier, sampler)
+    ms, t_wall, mark = timed_steps(wl, a, dev, stream, barrier, sampler)
     clocks = sampler.stop(mark)
-    launches_per_block = (_lib.launch_count() - launches0) / float(len(ms_blocks) + 1)       # pilot + repeats, all identical
-    ms = float(np.median(ms_blocks))
+    launches = _lib.launch_count() - launches0
+    if a.dump_outputs and rank == 0:
+        dump_outputs(wl, a.dump_outputs)
     value = N * world * a.steps / (ms * 1e-3)
     if world > 1:       # every rank's clock record, gathered
         allc = [None] * world
@@ -527,18 +535,16 @@ def run_ours(a):
         out = {"metric": "env steps/sec (+ DQN updates/sec), 500x500x100 city", "value": value, "unit": "env_steps/s",
                "updates_per_s": a.steps / (ms * 1e-3), "samples_per_s": a.steps * B * world / (ms * 1e-3),
                "n_gpus": world, "steps": a.steps, "warmup": max(a.warmup, 3), "ms_per_step": ms / a.steps,
-               "repeats": int(len(ms_blocks)), "block_ms_median": ms, "block_ms_min": float(ms_blocks.min()), "block_ms_max": float(ms_blocks.max()),
-               "timed_region_s": t_wall,
+               "timed_ms": ms, "timed_region_s": t_wall,
                "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
                "dtype": "f64 env state / f32 obs+learner", "data": "synthetic",
                "config": dict(config_dict(a, world), qnet_path=("tcgen05 3xTF32 (fp32-grade)" if tc_on else "fp32 CUDA cores"),
                               launch=("programmatic dependent launch" if a.pdl else "serialised")
                               + (", get_action+step fused" if (a.fuse and tc_on) else ""),
-                              timing="the %d-step block (barrier + synchronize both sides, CUDA events, max over ranks) repeated %d times; "
-                                     "value = median block" % (a.steps, len(ms_blocks))),
-               "clocks": clocks, "gpu_launches": int(round(launches_per_block)),
-               "gpu_launches_timed_region": int(round(launches_per_block * len(ms_blocks))),
-               "host_wall_ms_per_step": 1e3 * t_wall / (a.steps * len(ms_blocks))}
+                              timing="the %d timed steps as one block (barrier + synchronize both sides, CUDA events, max over ranks)"
+                                     % a.steps),
+               "clocks": clocks, "gpu_launches": int(launches),
+               "host_wall_ms_per_step": 1e3 * t_wall / a.steps}
 
     # ---- roofline pass: per-kernel CUDA-event time (rank 0's GPU; same workload, events between kernels)
     if rank == 0:
@@ -643,12 +649,14 @@ def run_ours(a):
     if not a.no_configs:
         subs = {}
         if world == 1:
-            a2 = argparse.Namespace(**vars(a)); a2.envs = a2.batch = 16384; a2.net, a2.algo = "vanet2", "dueling"; a2.min_seconds = 0.5
+            # a fixed count of its own: about 0.5 s at the 0.1 ms per step this config takes on one B200
+            a2 = argparse.Namespace(**vars(a)); a2.envs = a2.batch = 16384; a2.net, a2.algo = "vanet2", "dueling"; a2.steps = 5000
             subs["configs[2]"] = measure_config(a2, rank, world, local, None, dev, stream, barrier,
                                                 "16384 envs, DuelingDQN (VAnet2), buildings.xml obstacle set, 1xB200")
             subs["configs[4]"] = measure_sac(a, local, dev, stream, "16384 envs, SAC_Trainer continuous-action UAV (actor+2 critics), 1xB200")
         if world == 8:
-            a3 = argparse.Namespace(**vars(a)); a3.envs = a3.batch = 8192; a3.net, a3.algo = "qvalue3", "ddqn"; a3.min_seconds = 0.5
+            # about 0.5 s: this per-GPU shape takes 73 us per step on one B200, plus the gradient exchange
+            a3 = argparse.Namespace(**vars(a)); a3.envs = a3.batch = 8192; a3.net, a3.algo = "qvalue3", "ddqn"; a3.steps = 6000
             subs["configs[3]"] = measure_config(a3, rank, world, local, dist, dev, stream, barrier,
                                                 "65536 envs (8192/GPU), DDQN, replay buffer 1M/GPU, grad allreduce across 8xB200")
         if rank == 0 and subs:
@@ -668,6 +676,8 @@ def run_ours(a):
 
 if __name__ == "__main__":
     args = parse()
+    if args.steps is None:
+        args.steps = 200 if args.impl == "reference" else 25000
     if args.batch <= 0:
         args.batch = args.envs
     usable_cpus()                           # read the affinity mask before any OpenMP runtime can pin this thread
